@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- stereo pairs/s of the hot path (StereoJoin -> CBCA -> SGM -> post) on N B200s.
 
-Contract (driver): `python bench.py --gpus N --steps K --warmup W [--impl reference]`, one JSON
+Usage: `python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]`, one JSON
 line on stdout from rank 0.  A "step" = one stereo pair (BASELINE.json config 3: 370x1226, d=228,
 C=64 features, kitti-slow post-processing with CBCA x4 + 4-direction SGM) through the fused native
 pipeline, one pair per GPU per step (pairs shard over GPUs with no collective: weak scaling).
@@ -52,7 +52,22 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--small", action="store_true", help="tiny workload (debug only; not a valid bench line)")
     ap.add_argument("--workload", default="k228", choices=sorted(WORKLOADS))
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the disparity maps of the last timed step as DIR/<name>.npy (rank 0); "
+                         "the inputs depend only on the arguments, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(dirname, arrays):
+    """`arrays`: name -> tensor, written as float32 .npy files"""
+    import numpy as np
+
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 class ClockSampler:
@@ -465,6 +480,7 @@ def run_b200(args):
     # ---- same steps in the exact mode (every output bit-identical to the reference) --------------------
     sp.set_cbca_mode("exact")
     ms_exact = timed_steps(sp, dev_in, disp, K, 2, world)
+    disp_exact = disp.clone()
     # SURVEY.md 8(d) fast-mode bar on disp.bin: <= 1e-4 on >= (1 - 1e-4) of the pixels
     fast_diff_frac = float(((disp_fast - disp).abs() > 1e-4 * disp.abs().clamp(min=1.0)).float().mean().item())
     sp.set_cbca_mode("fast")
@@ -582,6 +598,9 @@ def run_b200(args):
         dist.barrier()
         dist.destroy_process_group()
     if out is not None:
+        if args.dump_outputs:
+            # the headline (default-mode) timed path and the exact mode's, each from its last timed step
+            dump_outputs(args.dump_outputs, {"disp": disp_fast, "disp_exact": disp_exact})
         os.write(json_fd, (json.dumps(out) + "\n").encode())
 
 
@@ -622,11 +641,13 @@ def run_reference(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(K):
-        refdriver.stereo_predict(shim, xb[i % 2], ft[i % 2], opt, cfg["D"])
+        disp = refdriver.stereo_predict(shim, xb[i % 2], ft[i % 2], opt, cfg["D"])
     e1.record()
     barrier_sync(world)
     ms = max_over_ranks(e0.elapsed_time(e1), world)
     clocks = sampler.stop()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"disp": disp.reshape(cfg["H"], cfg["W"])})
     if world > 1:
         import torch.distributed as dist
 
