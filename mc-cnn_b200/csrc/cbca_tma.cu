@@ -1,5 +1,7 @@
 // cbca_tma.cu -- cross-based cost aggregation with CONSTANT WORK PER PIXEL (adcensus.cbca, adcensus.cu:343-400)
 // for sm_100a: TMA-staged plane tiles, prefix sums along x, one column walk per thread.
+// This is the first generation.  Arms of up to 5 pixels go to the second generation (cbca_ws.cu, faster and more
+// accurate); this kernel is kept as the constant-work path for arms of 6-14 pixels behind mccnn_cbca_fast_pitched*.
 //
 // The reference gathers up to (2*L1-1)^2 taps per output.  The run of a support row depends on (d, row,
 // column) only, not on which output row uses it, so with I = inclusive prefix of the tile row
@@ -24,14 +26,13 @@
 //     ring of 2R + 2 rows; the output of row y is emitted R rows later from two ring reads.
 // Arms are pre-packed per image into H words (4L | 4(R-1) << 16) and V words (U << 8 | D << 24), lengths
 // relative to the pixel, so "max of left ends / min of right ends" is one packed 16-bit minimum.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "tma.cuh"
 
 namespace {
 
 constexpr int CT_TX = 128, CT_TY = 32, CT_NT = 256, CT_HO = CT_TY / 2;
+constexpr int CT_WB = 4;                   // rows per walk batch
 constexpr int CT_DCH = 20;                 // disparities per CTA (window width); the per-CTA staging of the arm windows is amortised over them
 constexpr int CT_WW = CT_TX + CT_DCH;      // pitch of the right-image arm windows
 
@@ -41,10 +42,10 @@ struct CTCfg {
 	static constexpr int HX = (HALO + 3) & ~3;         // left halo in columns: TMA needs a 16-byte aligned start along x
 	static constexpr int TH = CT_TY + 2 * R + 1;       // image rows y0 - HALO .. y0 + TY + R - 1
 	static constexpr int TWMIN = HX + CT_TX + R;       // image columns x0 - HX .. x0 + TX + R - 1
-	static constexpr int SEG = R <= 4 ? 28 : 20;       // the tile pitch is a multiple of 20 floats (16-byte rows for TMA, 5 per lane for the row scan)
+	static constexpr int SEG = 20;                     // the tile pitch is a multiple of 20 floats (16-byte rows for TMA, 5 per lane for the row scan)
 	static constexpr int NSEG = (TWMIN + SEG - 1) / SEG;
-	static constexpr int TWP = NSEG * SEG;             // tile pitch = TMA box width (140 / 160 floats)
-	static constexpr int RING = R <= 1 ? 4 : (R <= 7 ? 16 : 32);   // >= 2R + 2 rows of (T, N) per thread
+	static constexpr int TWP = NSEG * SEG;             // tile pitch = TMA box width (160 floats)
+	static constexpr int RING = 32;                    // >= 2R + 2 rows of (T, N) per thread
 	static constexpr int NWALK = 2 * R + CT_HO;        // rows a thread walks for its 16 outputs
 	static constexpr int TILE_BYTES = TH * TWP * 4;    // = bytes one TMA box delivers
 	static constexpr int STAGE_BYTES = (TILE_BYTES + 127) & ~127;
@@ -57,7 +58,7 @@ struct CTCfg {
 	static_assert(TWP <= 256 && TH <= 256, "TMA box limits");
 };
 
-template <int R, int WB>
+template <int R>
 __global__ void __launch_bounds__(CT_NT, (CTCfg<R>::SMEM <= 112 * 1024) ? 2 : 1)
 cbca_tma_kernel(const __grid_constant__ CUtensorMap tmap,
 		const uint32_t *__restrict__ a0h, const uint32_t *__restrict__ a0v,
@@ -213,14 +214,14 @@ cbca_tma_kernel(const __grid_constant__ CUtensorMap tmap,
 		float T = 0.0f;
 		int N = 0;
 		*reinterpret_cast<float2 *>(rgb) = make_float2(0.0f, __int_as_float(0));   // relative row 0: the excluded row of output 0
-		// rows in batches of WB: all the shared-memory reads of a batch are issued before its (short) serial part, so that
+		// rows in batches of CT_WB: all the shared-memory reads of a batch are issued before its (short) serial part, so that
 		// their latency overlaps (the kernel is latency-, not bandwidth-bound at 16 warps per SM)
 #pragma unroll
-		for (int b0 = 1; b0 <= NWALK; b0 += WB) {
-			uint32_t hw[WB], vw[WB];
-			float ph[WB], pl[WB];
+		for (int b0 = 1; b0 <= NWALK; b0 += CT_WB) {
+			uint32_t hw[CT_WB], vw[CT_WB];
+			float ph[CT_WB], pl[CT_WB];
 #pragma unroll
-			for (int i = 0; i < WB; i++) {
+			for (int i = 0; i < CT_WB; i++) {
 				const int rr = b0 + i;
 				if (rr <= NWALK) {
 					hw[i] = __vminu2(ah[rr - 1], wh[rr * CT_WW]);   // min of lengths = (max of left ends, min of right ends), :362-363
@@ -231,7 +232,7 @@ cbca_tma_kernel(const __grid_constant__ CUtensorMap tmap,
 				}
 			}
 #pragma unroll
-			for (int i = 0; i < WB; i++) {
+			for (int i = 0; i < CT_WB; i++) {
 				const int rr = b0 + i;
 				if (rr <= NWALK) {
 					const int L4 = hw[i] & 0xffffu, R4 = hw[i] >> 16;
@@ -241,7 +242,7 @@ cbca_tma_kernel(const __grid_constant__ CUtensorMap tmap,
 				}
 			}
 #pragma unroll
-			for (int i = 0; i < WB; i++) {
+			for (int i = 0; i < CT_WB; i++) {
 				const int rr = b0 + i;
 				if (rr > NWALK) continue;
 				const int L4 = hw[i] & 0xffffu, R4 = hw[i] >> 16;
@@ -310,7 +311,7 @@ __global__ void pack_arms_hv_kernel(const float *__restrict__ xc, uint32_t *__re
 	vw[id] = ((uint32_t)u << 8) | ((uint32_t)d << 24);
 }
 
-template <int R, int WB>
+template <int R>
 int launch_tma(const CUtensorMap &tm, const uint32_t *hv, const float *vol, float *out, int D, int H, int W, int ld, int direction,
 	       cudaStream_t s)
 {
@@ -319,16 +320,12 @@ int launch_tma(const CUtensorMap &tm, const uint32_t *hv, const float *vol, floa
 	int dev = 0;
 	cudaGetDevice(&dev);
 	if (!attr_done[dev & 63]) {
-		ADC_CUDA(cudaFuncSetAttribute(cbca_tma_kernel<R, WB>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
+		ADC_CUDA(cudaFuncSetAttribute(cbca_tma_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
 		attr_done[dev & 63] = true;
 	}
-	const char *env = getenv("ADCENSUS_CBCA_DCH");         // tuning knob, not part of the ABI
-	int dch = env ? atoi(env) : CT_DCH;
-	if (dch < 1) dch = 1;
-	if (dch > CT_DCH) dch = CT_DCH;
 	const long HW = (long)H * W;
-	dim3 grid(adc_div_up(W, CT_TX), adc_div_up(H, CT_TY), adc_div_up(D, dch));
-	cbca_tma_kernel<R, WB><<<grid, CT_NT, C::SMEM, s>>>(tm, hv, hv + 2 * HW, hv + HW, hv + 3 * HW, vol, out, D, H, W, ld, direction, dch);
+	dim3 grid(adc_div_up(W, CT_TX), adc_div_up(H, CT_TY), adc_div_up(D, CT_DCH));
+	cbca_tma_kernel<R><<<grid, CT_NT, C::SMEM, s>>>(tm, hv, hv + 2 * HW, hv + HW, hv + 3 * HW, vol, out, D, H, W, ld, direction, CT_DCH);
 	ADC_CHECK_LAUNCH();
 	return 0;
 }
@@ -347,16 +344,11 @@ int adc_pack_arms_hv(const float *xc, uint32_t *hv, int which, int H, int W, cud
 	return 0;
 }
 
-// second-generation kernel for short arms (cbca_ws.cu); ADCENSUS_CBCA_WS=0 keeps the first-generation one
+// second-generation kernel for short arms (cbca_ws.cu)
 int adc_cbca_ws_max_halo();
 void adc_cbca_ws_box(int halo, int *box_w, int *box_h);
 int adc_cbca_ws(const CUtensorMap *tm, const uint32_t *hv, const float *vol, float *out, int D, int H, int W, int ld, int direction,
 		int halo, cudaStream_t s);
-static bool use_ws(int halo)
-{
-	static const int ws = getenv("ADCENSUS_CBCA_WS") ? atoi(getenv("ADCENSUS_CBCA_WS")) : 1;
-	return ws && halo <= adc_cbca_ws_max_halo();
-}
 
 // largest support radius (longest arm - 1) the constant-work kernel is instantiated for
 int adc_cbca_tma_max_halo() { return 13; }
@@ -364,9 +356,7 @@ int adc_cbca_tma_max_halo() { return 13; }
 // box of the tensor map a volume needs for support radius `halo` (= longest arm - 1)
 void adc_cbca_tma_box(int halo, int *box_w, int *box_h)
 {
-	if (use_ws(halo)) adc_cbca_ws_box(halo, box_w, box_h);
-	else if (halo <= 1) { *box_w = CTCfg<1>::TWP; *box_h = CTCfg<1>::TH; }
-	else if (halo <= 4) { *box_w = CTCfg<4>::TWP; *box_h = CTCfg<4>::TH; }
+	if (halo <= adc_cbca_ws_max_halo()) adc_cbca_ws_box(halo, box_w, box_h);
 	else if (halo <= 8) { *box_w = CTCfg<8>::TWP; *box_h = CTCfg<8>::TH; }
 	else { *box_w = CTCfg<13>::TWP; *box_h = CTCfg<13>::TH; }
 }
@@ -375,16 +365,9 @@ void adc_cbca_tma_box(int halo, int *box_w, int *box_h)
 int adc_cbca_tma(const CUtensorMap *tm, const uint32_t *hv, const float *vol, float *out, int D, int H, int W, int ld, int direction,
 		 int halo, cudaStream_t s)
 {
-	if (use_ws(halo)) return adc_cbca_ws(tm, hv, vol, out, D, H, W, ld, direction, halo, s);
-	if (halo <= 1) return launch_tma<1, 4>(*tm, hv, vol, out, D, H, W, ld, direction, s);
-	if (halo <= 4) {
-		static const int wb = getenv("ADCENSUS_CBCA_WB") ? atoi(getenv("ADCENSUS_CBCA_WB")) : 4;   // tuning knob (rows per walk batch)
-		if (wb == 6) return launch_tma<4, 6>(*tm, hv, vol, out, D, H, W, ld, direction, s);
-		if (wb == 8) return launch_tma<4, 8>(*tm, hv, vol, out, D, H, W, ld, direction, s);
-		return launch_tma<4, 4>(*tm, hv, vol, out, D, H, W, ld, direction, s);
-	}
-	if (halo <= 8) return launch_tma<8, 4>(*tm, hv, vol, out, D, H, W, ld, direction, s);
-	if (halo <= 13) return launch_tma<13, 4>(*tm, hv, vol, out, D, H, W, ld, direction, s);
+	if (halo <= adc_cbca_ws_max_halo()) return adc_cbca_ws(tm, hv, vol, out, D, H, W, ld, direction, halo, s);
+	if (halo <= 8) return launch_tma<8>(*tm, hv, vol, out, D, H, W, ld, direction, s);
+	if (halo <= 13) return launch_tma<13>(*tm, hv, vol, out, D, H, W, ld, direction, s);
 	return ADCENSUS_ELIMIT;
 }
 

@@ -1,67 +1,61 @@
 // cbca_ws.cu -- constant-work cross-based cost aggregation (adcensus.cbca, adcensus.cu:343-400), second generation:
-// warp-specialised, three-stage TMA pipeline, vertical sums in registers.
+// warp-specialised, three-stage TMA pipeline, running sums down the column in a per-thread ring.
 //
 // Same decomposition as cbca_tma.cu -- the run of a support row depends on (d, row, column) only, so with I the
 // inclusive prefix of a tile row
-//     S(r, x) = I(r, x + R_ - 1) - I(r, x - L)          sum of the run (x - L, x + R_) of row r        (:362-369)
-//     out(y, x) = sum_{r = y-U+1}^{y+Dn-1} S(r, x) / sum of the run lengths                            (:361, :373)
-// -- but the work is split by ROLE instead of by phase, and the vertical part no longer goes through memory:
+//     S(r, x)   = I(r, x + R_ - 1) - I(r, x - L)                                 sum of the run (x - L, x + R_)  (:362-369)
+//     out(y, x) = (T(y + Dn - 1, x) - T(y - U, x)) / (N(y + Dn - 1, x) - N(y - U, x))                            (:361, :373)
+// with T, N the running sums of S and of the run lengths down the column -- but the work is split by ROLE instead of
+// by phase:
 //   * one PRODUCER thread keeps three plane tiles in flight (cp.async.bulk.tensor.3d, one box of 144 x (64 + 2R + 1)
 //     floats per disparity, zero-filled outside the image) behind full / ready / empty mbarriers;
 //   * four PREFIX warps turn each landed tile into row prefixes in place: two tile rows per warp instruction
 //     (16 lanes x 9 consecutive columns each, bank-conflict free at the 144-float pitch), two such pairs interleaved
-//     (the scan is a chain of dependent adds and shuffles), a 4-step shuffle scan,
-//     optionally centred on one value per tile so that |I| stays a random walk instead of growing with the mean
-//     (less cancellation in the differences);
+//     (the scan is a chain of dependent adds and shuffles), a 4-step shuffle scan.  The prefixes are centred: one
+//     value per tile (its mid pixel) is subtracted first, so that |I| stays a random walk instead of growing with the
+//     mean of the plane (less cancellation in the differences); the walkers add it back to every output;
 //   * eight WALKER warps: thread = (column, half of the 64 output rows).  A thread walks 32 + 2R tile rows once;
 //     per row one LDS of the right image's arms, one packed 16-bit minimum against its own column's arms (registers
-//     for the whole disparity chunk), two prefix look-ups -> (S, run length) as a packed f32x2 that stays in
-//     registers for the 2R + 1 outputs whose vertical range can contain the row.  An output is 2R + 1 predicated
-//     add.rn.f32x2 in ascending row order (the reference's row order), a reciprocal with one Newton step, one store.
-//     No per-thread ring in shared memory, no block-wide barrier in the steady state.
-// Compared with cbca_tma.cu (32-row tiles, 2 CTAs per SM, prefix and walk as barrier-separated phases, (T, N) ring in
-// shared memory): 40 % fewer shared-memory wavefronts per output, 64-row tiles (halo overhead 1.25 instead of 1.4 / 1.5),
-// and no cancellation in the vertical direction.  NOT bit-exact by construction (1e-4 contract; measured ~1e-7).
+//     for the whole disparity chunk), two prefix look-ups -> (S, run length), added as a packed f32x2 to the running
+//     (T, N) pair, which goes into a per-thread ring of 16 rows in shared memory.  The output of row y is emitted
+//     R rows later as the difference of two ring entries, a reciprocal with one Newton step, one store.
+//     No block-wide barrier in the steady state.
+// Compared with cbca_tma.cu (32-row tiles, 2 CTAs per SM, prefix and walk as barrier-separated phases): 40 % fewer
+// shared-memory wavefronts per output, 64-row tiles (halo overhead 1.25 instead of 1.4 / 1.5), and centred prefixes.
+// NOT bit-exact by construction (1e-4 contract; measured ~1e-7).
 // Arms up to 5 pixels (R <= 4, the KITTI presets); longer arms stay on cbca_tma.cu / the exact kernels.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "tma.cuh"
 
 namespace {
 
 constexpr int WS_TX = 128, WS_TY = 64;
-__host__ __device__ constexpr int ws_nwt(int ho) { return WS_TX * (WS_TY / ho); }                  // walker threads: column x row group
-// walkers + prefix warps + one producer warp; the 512-walker form has no producer warp (prefix warp 0 issues the TMA) so that the
-// block stays within 640 threads = 96 registers per thread
-__host__ __device__ constexpr int ws_nt(int npw, int ho) { return ws_nwt(ho) + 32 * npw + (ho < 32 ? 0 : 32); }
+constexpr int WS_HO = 32;                   // output rows per walker thread
+constexpr int WS_NWT = WS_TX * (WS_TY / WS_HO);   // walker threads: column x row group
+constexpr int WS_NPW = 4;                   // prefix warps
+constexpr int WS_NT = WS_NWT + 32 * WS_NPW + 32;  // walkers + prefix warps + one producer warp
+constexpr int WS_NST = 3;                   // tile stages
+constexpr int WS_RING = 16;                 // rows of (T, N) per walker thread (>= 2R + 2; a power of two: cheap wrap)
 constexpr int WS_DCH = 20;                  // max disparities per CTA
 constexpr int WS_WW = WS_TX + WS_DCH;       // pitch of the right-image arm windows
 constexpr int WS_TWP = 144;                 // tile pitch = TMA box width: 16 lanes x 9 columns, = 16 (mod 32)
 
-// LEAN: two tile stages and a 16-bit H-word window: 150 KB instead of 216 KB of shared memory, which leaves room for an SGM /
-// transpose CTA of the other direction (or lane) on the same SM -- the issue-bound walk and the HBM-bound scans overlap
-template <int R, int HO, bool LEAN>
+template <int R>
 struct WSCfg {
-	static constexpr int NST = LEAN ? 2 : 3;           // tile stages
 	static constexpr int HALO = R + 1;                 // the prefix differences index the first EXCLUDED pixel
 	static constexpr int HX = (HALO + 3) & ~3;         // left halo in columns (TMA: 16-byte aligned start along x)
 	static constexpr int TH = WS_TY + 2 * R + 1;       // image rows y0 - HALO .. y0 + TY + R - 1
-	static constexpr int NWALK = 2 * R + HO;           // rows a thread walks for its HO outputs
-	static constexpr int NWT = ws_nwt(HO);
-	static constexpr bool H16 = HO < 32 || LEAN;       // narrow the H-word window to 16 bits (shared-memory budget)
+	static constexpr int NWALK = 2 * R + WS_HO;        // rows a thread walks for its WS_HO outputs
 	static constexpr int TILE_BYTES = TH * WS_TWP * 4; // bytes one TMA box delivers
 	static constexpr int STAGE_BYTES = (TILE_BYTES + 127) & ~127;
-	static constexpr int OFF_WINH = NST * STAGE_BYTES;
-	static constexpr int OFF_WINV = OFF_WINH + ((TH * WS_WW * (H16 ? 2 : 4) + 15) & ~15);
+	static constexpr int OFF_WINH = WS_NST * STAGE_BYTES;
+	static constexpr int OFF_WINV = OFF_WINH + ((TH * WS_WW * 4 + 15) & ~15);
 	static constexpr int OFF_MU = OFF_WINV + ((WS_TY * WS_WW * 2 + 15) & ~15);
 	static constexpr int OFF_BAR = OFF_MU + 16;
-	static constexpr int OFF_RING = OFF_BAR + ((3 * NST * 8 + 15) & ~15);   // VMODE 2 only: [RING][NWT] (T, N) per thread
-	static constexpr int RING = (HO < 32 || LEAN) ? 2 * R + 2 : 16;   // a power of two where the budget allows (cheaper wrap)
-	static constexpr int SMEM_NORING = OFF_RING;
-	static constexpr int SMEM_RING = OFF_RING + RING * NWT * 8;
-	static_assert(SMEM_RING <= 232448, "shared memory budget");
-	static_assert(RING >= 2 * R + 2, "ring too small");
+	static constexpr int OFF_RING = OFF_BAR + ((3 * WS_NST * 8 + 15) & ~15);   // [WS_RING][WS_NWT] (T, N) per thread
+	static constexpr int SMEM = OFF_RING + WS_RING * WS_NWT * 8;
+	static_assert(SMEM <= 232448, "shared memory budget");
+	static_assert(WS_RING >= 2 * R + 2, "ring too small");
 	static_assert(HX + WS_TX + R <= WS_TWP, "tile pitch too small");
 	static_assert(TH <= 256, "TMA box limit");
 };
@@ -75,16 +69,6 @@ __device__ __forceinline__ unsigned long long ws_pack2(float lo, float hi)
 	unsigned long long r;
 	asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
 	return r;
-}
-__device__ __forceinline__ void ws_unpack2(unsigned long long v, float &lo, float &hi)
-{
-	asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
-}
-__device__ __forceinline__ unsigned long long ws_fma2(unsigned long long a, unsigned long long b, unsigned long long c)
-{
-	unsigned long long d;
-	asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
-	return d;
 }
 __device__ __forceinline__ unsigned long long ws_add2(unsigned long long a, unsigned long long b)
 {
@@ -114,27 +98,22 @@ __device__ __forceinline__ void ws_copy_planes(const float *__restrict__ vol, fl
 	}
 }
 
-// CENTER: subtract one value per tile (the tile's mid pixel, 0 when that is not finite) before the row prefix and add
-// it back per run (mu * length): the prefixes then carry deviations instead of the level of the plane.
-// VMODE: how an output gathers its rows y - U + 1 .. y + Dn - 1:
-//   1  2R + 1 fma.rn.f32x2 with a 0/1 float mask per row (mask = saturate(arm - j): one FADD.SAT)
-//   2  running (T, N) down the column in a per-thread shared-memory ring, output = difference of two entries (fewest
-//      instructions, most shared-memory traffic); with CENTER the running sums carry deviations only
-// (predicated add.rn.f32x2 was tried first: ptxas turns each into FADD2 + 2 SEL, 70 instructions per output)
-template <int R, int WB, bool CENTER, int VMODE, int WS_NPW, int WS_HO, bool LEAN>
-__global__ void __launch_bounds__(ws_nt(WS_NPW, WS_HO), 1)
+// Centring: the prefix warps subtract one value per tile (the tile's mid pixel, 0 when that is not finite) before the row
+// prefix; the running sums then carry deviations only, and the walkers add the value back to each quotient.
+// (Two other ways for an output to gather its rows were measured slower: 2R + 1 predicated add.rn.f32x2, which ptxas
+// turns into FADD2 + 2 SEL each, and 2R + 1 fma.rn.f32x2 with 0/1 masks.)
+template <int R, int WB>
+__global__ void __launch_bounds__(WS_NT, 1)
 cbca_ws_kernel(const __grid_constant__ CUtensorMap tmap,
 	       const uint32_t *__restrict__ a0h, const uint32_t *__restrict__ a0v,
 	       const uint32_t *__restrict__ a1h, const uint32_t *__restrict__ a1v,
 	       const float *__restrict__ vol, float *__restrict__ out,
 	       int D, int H, int W, int ld, int direction, int dch)
 {
-	using C = WSCfg<R, WS_HO, LEAN>;
-	constexpr int WS_NT = ws_nt(WS_NPW, WS_HO), WS_NWT = C::NWT, WS_NST = C::NST;
+	using C = WSCfg<R>;
 	constexpr int HALO = C::HALO, HX = C::HX, TH = C::TH, NWALK = C::NWALK, TWP = WS_TWP;
 	extern __shared__ __align__(128) unsigned char ws_smem[];
-	uint32_t *winH = reinterpret_cast<uint32_t *>(ws_smem + C::OFF_WINH);   // [TH][WS_WW] right-image H words (32-bit form)
-	uint16_t *winH16 = reinterpret_cast<uint16_t *>(ws_smem + C::OFF_WINH); // same, narrowed: 4L | 4(R-1) << 8
+	uint32_t *winH = reinterpret_cast<uint32_t *>(ws_smem + C::OFF_WINH);   // [TH][WS_WW] right-image H words
 	uint16_t *winV = reinterpret_cast<uint16_t *>(ws_smem + C::OFF_WINV);   // [WS_TY][WS_WW] right-image U | D << 8
 	float *mus = reinterpret_cast<float *>(ws_smem + C::OFF_MU);            // [WS_NST] centre value of the stage's tile
 	uint64_t *bar_full = reinterpret_cast<uint64_t *>(ws_smem + C::OFF_BAR);   // TMA landed
@@ -166,8 +145,7 @@ cbca_ws_kernel(const __grid_constant__ CUtensorMap tmap,
 	}
 	__syncthreads();
 
-	constexpr bool MERGED = WS_HO < 32;                // no producer warp: prefix warp 0, lane 0 issues the TMA
-	constexpr int W_PROD = MERGED ? WS_NWT / 32 : WS_NWT / 32 + WS_NPW;   // warp whose lane 0 issues the TMA
+	constexpr int W_PROD = WS_NWT / 32 + WS_NPW;       // warp whose lane 0 issues the TMA
 	if (warp == W_PROD && lane == 0) {                 // the first tiles fly while the arm windows are staged
 #pragma unroll
 		for (int s = 0; s < WS_NST; s++)
@@ -190,14 +168,9 @@ cbca_ws_kernel(const __grid_constant__ CUtensorMap tmap,
 				const int j = lane + 32 * m, xx = a1x0 + j;
 				if (j < WS_WW) {
 					const bool ok = rowok && xx >= 0 && xx < W;
-					if (C::H16) {
-						const uint32_t v = ok ? __ldg(grow + xx) : 0u;
-						winH16[r * WS_WW + j] = (uint16_t)((v & 255u) | ((v >> 8) & 0xff00u));
-					} else {
-						const unsigned dst = (unsigned)__cvta_generic_to_shared(winH + r * WS_WW + j);
-						const int nbytes = ok ? 4 : 0;
-						asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(dst), "l"(grow + (ok ? xx : 0)), "r"(nbytes));
-					}
+					const unsigned dst = (unsigned)__cvta_generic_to_shared(winH + r * WS_WW + j);
+					const int nbytes = ok ? 4 : 0;
+					asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(dst), "l"(grow + (ok ? xx : 0)), "r"(nbytes));
 				}
 			}
 		}
@@ -221,7 +194,7 @@ cbca_ws_kernel(const __grid_constant__ CUtensorMap tmap,
 		asm volatile("bar.sync 2, %0;" ::"n"(WS_NWT) : "memory");   // windows visible to the walkers
 	}
 
-	if (!MERGED && warp == W_PROD) {
+	if (warp == W_PROD) {
 		// ---------------------------------------------------------------- producer
 		if (lane == 0) {
 			for (int dd = WS_NST; dd < nproc; dd++) {
@@ -247,16 +220,13 @@ cbca_ws_kernel(const __grid_constant__ CUtensorMap tmap,
 			// sum would carry them along the row: count them as 0.
 			const bool scrub = direction < 0 ? (x0 - HX - d < 0) : (x0 - HX + TWP + d > W);
 			mbar_wait(&bar_full[s], (dd / WS_NST) & 1);
-			float mu = 0.0f;
-			if (CENTER) {
-				const float m = P[(HALO + WS_TY / 2) * TWP + HX + WS_TX / 2];
-				mu = (fabsf(m) <= 3.0e38f) ? m : 0.0f;               // finite (NaN and inf fail the compare)
-				if (pw == 0 && lane == 0) mus[s] = mu;
-				asm volatile("bar.sync 1, %0;" ::"n"(32 * WS_NPW) : "memory");   // every prefix warp has read it before any row is rewritten
-			}
+			const float m = P[(HALO + WS_TY / 2) * TWP + HX + WS_TX / 2];
+			const float mu = (fabsf(m) <= 3.0e38f) ? m : 0.0f;   // finite (NaN and inf fail the compare)
+			if (pw == 0 && lane == 0) mus[s] = mu;
+			asm volatile("bar.sync 1, %0;" ::"n"(32 * WS_NPW) : "memory");   // every prefix warp has read it before any row is rewritten
 			// two independent row pairs per iteration (the scan of one is a chain of dependent adds and shuffles: a single
 			// pair per iteration left the prefix warps latency-bound and the walkers waiting for them)
-			constexpr int UP = WS_NPW <= 3 ? 4 : 2;         // independent row pairs per iteration
+			constexpr int UP = 2;
 			for (int pr0 = pw; pr0 < (TH + 1) / 2; pr0 += UP * WS_NPW) {
 				float v[UP][EPL];
 				float *row[UP];
@@ -271,10 +241,8 @@ cbca_ws_kernel(const __grid_constant__ CUtensorMap tmap,
 				}
 #pragma unroll
 				for (int u = 0; u < UP; u++) {
-					if (CENTER) {
 #pragma unroll
-						for (int i = 0; i < EPL; i++) v[u][i] -= mu;
-					}
+					for (int i = 0; i < EPL; i++) v[u][i] -= mu;
 					if (scrub) {
 #pragma unroll
 						for (int i = 0; i < EPL; i++) v[u][i] = v[u][i] == v[u][i] ? v[u][i] : 0.0f;
@@ -309,17 +277,6 @@ cbca_ws_kernel(const __grid_constant__ CUtensorMap tmap,
 			fence_proxy_async_smem();                      // generic writes of this stage before its next TMA refill
 			__syncwarp();
 			if (lane == 0) mbar_arrive(&bar_ready[s]);
-			if (MERGED && pw == 0) {
-				// producer duty AFTER this plane's prefixes are published: plane dd + 2 goes into the stage the walkers
-				// release when they finish plane dd - 1 (they are walking it now; plane dd is already waiting for them)
-				if (lane == 0 && dd >= 1 && dd + WS_NST - 1 < nproc) {
-					const int nx = dd + WS_NST - 1, s2 = nx % WS_NST;
-					mbar_wait(&bar_empty[s2], ((nx / WS_NST) - 1) & 1);
-					mbar_arrive_expect_tx(&bar_full[s2], C::TILE_BYTES);
-					tma_load_3d(ws_smem + s2 * C::STAGE_BYTES, &tmap, x0 - HX, y0 - HALO, d0 + nx, &bar_full[s2]);
-				}
-				__syncwarp();
-			}
 		}
 		return;
 	}
@@ -350,21 +307,19 @@ cbca_ws_kernel(const __grid_constant__ CUtensorMap tmap,
 		const bool valid_col = x < W && xs >= 0 && xs < W;
 		const int off = (x0 + sh) - a1x0;                 // window column of tile column 0
 		mbar_wait(&bar_ready[s], (dd / WS_NST) & 1);
-		const float mu = CENTER ? mus[s] : 0.0f;
+		const float mu = mus[s];
 
 		// column walk: relative row rr <-> tile row 32h + rr <-> image row yb - HALO + rr
 		const char *Pc = reinterpret_cast<const char *>(P + (WS_HO * h) * TWP + c + HX);   // own pixel's prefix entry, relative row 0
 		const uint32_t *wh = winH + (WS_HO * h) * WS_WW + c + off;
-		const uint16_t *wh16 = winH16 + (WS_HO * h) * WS_WW + c + off;
 		const uint16_t *wv = winV + (WS_HO * h) * WS_WW + c + off;
 		char *po = reinterpret_cast<char *>(out + ((long)d * H + yb) * ld + x);
 		const long ldb = (long)ld * 4;
 		const int nst = valid_col ? nv : 0;                          // rows this thread stores from the walk
-		unsigned long long sn[NWALK + 1];                            // (S, run length) of relative rows 1 .. NWALK
-		constexpr int RROW = WS_NWT * 8;                             // ring row pitch in bytes (VMODE 2)
+		constexpr int RROW = WS_NWT * 8;                             // ring row pitch in bytes
 		char *rgb = reinterpret_cast<char *>(ws_smem + C::OFF_RING) + tid * 8;
 		unsigned long long run = ws_pack2(0.0f, 0.0f);
-		if (VMODE == 2) *reinterpret_cast<unsigned long long *>(rgb) = run;   // relative row 0: the excluded row of output 0
+		*reinterpret_cast<unsigned long long *>(rgb) = run;          // relative row 0: the excluded row of output 0
 		// rows in batches of WB: all the shared-memory reads of a batch are issued before its arithmetic
 #pragma unroll
 		for (int b0 = 1; b0 <= NWALK; b0 += WB) {
@@ -374,8 +329,7 @@ cbca_ws_kernel(const __grid_constant__ CUtensorMap tmap,
 			for (int i = 0; i < WB; i++) {
 				const int rr = b0 + i;
 				if (rr <= NWALK) {
-					const uint32_t wr = C::H16 ? __byte_perm((uint32_t)wh16[rr * WS_WW], 0u, 0x4140) : wh[rr * WS_WW];
-					hw[i] = __vminu2(ah[rr - 1], wr);               // min of lengths = (max of left ends, min of right ends), :362-363
+					hw[i] = __vminu2(ah[rr - 1], wh[rr * WS_WW]);   // min of lengths = (max of left ends, min of right ends), :362-363
 					if (rr >= 2 * R + 1) {
 						const int k = rr - 2 * R - 1;
 						vw[i] = __vminu2(av[k], __byte_perm((uint32_t)wv[k * WS_WW], 0u, 0x1404));   // :359-360
@@ -399,65 +353,29 @@ cbca_ws_kernel(const __grid_constant__ CUtensorMap tmap,
 				const int L4 = hw[i] & 0xffffu, R4 = hw[i] >> 16;
 				// run length L + R_ - 1 = (L4 + R4) / 4 as a float without a conversion: (2^23 + m) / 4 - 2^21, all exact
 				const float nf = fmaf(__int_as_float(0x4B000000 + L4 + R4), 0.25f, -2097152.0f);   // :368
-				float S = ph[i] - pl[i];                               // sum of the run (x - L, x + R_), :364-367
-				if (CENTER && VMODE != 2) S = fmaf(mu, nf, S);
-				if (VMODE == 2) {
-					run = ws_add2(run, ws_pack2(S, nf));
-					*reinterpret_cast<unsigned long long *>(rgb + (rr % C::RING) * RROW) = run;
-				} else {
-					sn[rr] = ws_pack2(S, nf);
-				}
+				const float S = ph[i] - pl[i];                         // sum of the run (x - L, x + R_), :364-367
+				run = ws_add2(run, ws_pack2(S, nf));
+				*reinterpret_cast<unsigned long long *>(rgb + (rr % WS_RING) * RROW) = run;
 				if (rr >= 2 * R + 1) {
 					const int k = rr - 2 * R - 1;                    // output row yb + k = relative row HALO + k = k + R + 1
 					const unsigned U8 = vw[i] & 0xffffu, D8 = vw[i] >> 16;   // U << 8, Dn << 8
-					float T, N;
-					if (VMODE == 2) {
-						constexpr int RING = C::RING, RB = RING * RROW;
-						constexpr int SC = RROW / 256;                 // U8 = U << 8: U8 * SC = U * RROW
-						const int rk = HALO + k;
-						// rows y - U + 1 .. y + Dn - 1 (:361): run(rk + Dn - 1) - run(rk - U); the ring index wraps only
-						// where the (compile-time) row position says it can
-						constexpr bool POW2 = (RING & (RING - 1)) == 0;
-						const int sb = (rk - 1) % RING, sb2 = rk % RING;
-						int oh = D8 * SC + sb * RROW;
-						if (sb + R + 1 >= RING) {
-							if (POW2) oh &= RB - 1;
-							else oh = oh >= RB ? oh - RB : oh;
-						}
-						int ol = sb2 * RROW - U8 * SC;
-						if (sb2 - R - 1 < 0) {
-							if (POW2) ol = (ol + RB) & (RB - 1);
-							else ol = ol < 0 ? ol + RB : ol;
-						}
-						const float2 a = *reinterpret_cast<const float2 *>(rgb + oh), b = *reinterpret_cast<const float2 *>(rgb + ol);
-						T = a.x - b.x;
-						N = a.y - b.y;
-					} else {
-						// ascending rows like the reference
-						unsigned long long acc = ws_pack2(0.0f, 0.0f);
-						{
-							// arm lengths as floats without a conversion: (2^23 + 256 a) / 256 - 2^15
-							const float Uf = fmaf(__int_as_float(0x4B000000 + U8), 0.00390625f, -32768.0f);
-							const float Df = fmaf(__int_as_float(0x4B000000 + D8), 0.00390625f, -32768.0f);
-#pragma unroll
-							for (int j = R; j >= 1; j--) {
-								const float m = __saturatef(Uf - (float)j);   // 1 iff U > j
-								acc = ws_fma2(sn[k + R + 1 - j], ws_pack2(m, m), acc);
-							}
-							acc = ws_add2(acc, sn[k + R + 1]);
-#pragma unroll
-							for (int j = 1; j <= R; j++) {
-								const float m = __saturatef(Df - (float)j);   // 1 iff Dn > j
-								acc = ws_fma2(sn[k + R + 1 + j], ws_pack2(m, m), acc);
-							}
-						}
-						ws_unpack2(acc, T, N);
-					}
+					constexpr int RB = WS_RING * RROW;
+					constexpr int SC = RROW / 256;                 // U8 = U << 8: U8 * SC = U * RROW
+					const int rk = HALO + k;
+					// rows y - U + 1 .. y + Dn - 1 (:361): run(rk + Dn - 1) - run(rk - U); the ring index wraps only
+					// where the (compile-time) row position says it can
+					const int sb = (rk - 1) % WS_RING, sb2 = rk % WS_RING;
+					int oh = D8 * SC + sb * RROW;
+					if (sb + R + 1 >= WS_RING) oh &= RB - 1;
+					int ol = sb2 * RROW - U8 * SC;
+					if (sb2 - R - 1 < 0) ol = (ol + RB) & (RB - 1);
+					const float2 a = *reinterpret_cast<const float2 *>(rgb + oh), b = *reinterpret_cast<const float2 *>(rgb + ol);
+					const float T = a.x - b.x, N = a.y - b.y;
 					float rc;
 					asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rc) : "f"(N));   // count >= 1
 					float q = T * rc;
 					q = fmaf(fmaf(-q, N, T), rc, q);                     // one Newton step: T / N to the last bit or so (:373)
-					if (CENTER && VMODE == 2) q += mu;
+					q += mu;
 					asm volatile("{\n\t.reg .pred p;\n\tsetp.lt.s32 p, %2, %3;\n\t@p st.global.f32 [%0], %1;\n\t}" ::"l"(po), "f"(q), "r"(k), "r"(nst)
 						     : "memory");
 					po += ldb;
@@ -480,26 +398,22 @@ cbca_ws_kernel(const __grid_constant__ CUtensorMap tmap,
 	}
 }
 
-template <int R, int WB, bool CENTER, int VMODE, int NPW, int HO, bool LEAN>
+template <int R, int WB>
 int launch_ws(const CUtensorMap &tm, const uint32_t *hv, const float *vol, float *out, int D, int H, int W, int ld, int direction,
 	      cudaStream_t s)
 {
-	using C = WSCfg<R, HO, LEAN>;
-	constexpr int smem = VMODE == 2 ? C::SMEM_RING : C::SMEM_NORING;
+	using C = WSCfg<R>;
 	static bool attr_done[64] = {false};
 	int dev = 0;
 	cudaGetDevice(&dev);
 	if (!attr_done[dev & 63]) {
-		ADC_CUDA(cudaFuncSetAttribute(cbca_ws_kernel<R, WB, CENTER, VMODE, NPW, HO, LEAN>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+		ADC_CUDA(cudaFuncSetAttribute(cbca_ws_kernel<R, WB>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
 		attr_done[dev & 63] = true;
 	}
-	static const int dch_env = getenv("ADCENSUS_CBCA_DCH") ? atoi(getenv("ADCENSUS_CBCA_DCH")) : 0;   // tuning knob, not part of the ABI
-	int dch = dch_env > 0 ? dch_env : WS_DCH;
-	if (dch > WS_DCH) dch = WS_DCH;
-	dch = adc_div_up(D, adc_div_up(D, dch));               // equal chunks (19 x 12 at D = 228)
+	const int dch = adc_div_up(D, adc_div_up(D, WS_DCH));   // equal chunks (19 x 12 at D = 228)
 	const long HW = (long)H * W;
 	dim3 grid(adc_div_up(W, WS_TX), adc_div_up(H, WS_TY), adc_div_up(D, dch));
-	cbca_ws_kernel<R, WB, CENTER, VMODE, NPW, HO, LEAN><<<grid, ws_nt(NPW, HO), smem, s>>>(tm, hv, hv + 2 * HW, hv + HW, hv + 3 * HW, vol, out, D, H, W, ld, direction, dch);
+	cbca_ws_kernel<R, WB><<<grid, WS_NT, C::SMEM, s>>>(tm, hv, hv + 2 * HW, hv + HW, hv + 3 * HW, vol, out, D, H, W, ld, direction, dch);
 	ADC_CHECK_LAUNCH();
 	return 0;
 }
@@ -512,38 +426,14 @@ int adc_cbca_ws_max_halo() { return 4; }
 void adc_cbca_ws_box(int halo, int *box_w, int *box_h)
 {
 	*box_w = WS_TWP;
-	*box_h = halo <= 1 ? WSCfg<1, 32, false>::TH : WSCfg<4, 32, false>::TH;
+	*box_h = halo <= 1 ? WSCfg<1>::TH : WSCfg<4>::TH;
 }
 
 // hv: packed arms (adc_pack_arms_hv); tm: tensor map of `vol` with the box of adc_cbca_ws_box(halo)
 int adc_cbca_ws(const CUtensorMap *tm, const uint32_t *hv, const float *vol, float *out, int D, int H, int W, int ld, int direction,
 		int halo, cudaStream_t s)
 {
-	// Tuning knobs (environment, read once; not part of the ABI).  Defaults = the fastest measured on B200 at the bench size
-	// that also keeps the disparity map inside the 1e-4-of-the-pixels bar: running sums in the ring, centred (VMODE 2,
-	// CENTER 1: 0.38 ms / iteration, 1.5e-5 of the pixels differ); VMODE 1 sums every row range tap by tap (0.39 ms, 9e-6).
-	static const int center = getenv("ADCENSUS_CBCA_CENTER") ? atoi(getenv("ADCENSUS_CBCA_CENTER")) : 1;
-	static const int vmode = getenv("ADCENSUS_CBCA_VMODE") ? atoi(getenv("ADCENSUS_CBCA_VMODE")) : 2;
-	static const int npw = getenv("ADCENSUS_CBCA_NPW") ? atoi(getenv("ADCENSUS_CBCA_NPW")) : 4;
-#define WS_GO(R_, WB_, C_, V_, N_, HO_) return launch_ws<R_, WB_, C_, V_, N_, HO_, false>(*tm, hv, vol, out, D, H, W, ld, direction, s)
-	static const int ho = getenv("ADCENSUS_CBCA_HO") ? atoi(getenv("ADCENSUS_CBCA_HO")) : 32;
-	if (halo <= 1) {
-		if (vmode == 2) { if (center) WS_GO(1, 6, true, 2, 4, 32); else WS_GO(1, 6, false, 2, 4, 32); }
-		if (center) WS_GO(1, 6, true, 1, 4, 32); else WS_GO(1, 6, false, 1, 4, 32);
-	}
-	if (halo <= 4) {
-		static const int lean = getenv("ADCENSUS_CBCA_LEAN") ? atoi(getenv("ADCENSUS_CBCA_LEAN")) : 0;
-		if (lean && vmode == 2 && center) return launch_ws<4, 4, true, 2, 4, 32, true>(*tm, hv, vol, out, D, H, W, ld, direction, s);
-		if (ho == 16) {                                    // 16 walker warps (column x quarter), ring mode only
-			if (center) WS_GO(4, 4, true, 2, 3, 16); else WS_GO(4, 4, false, 2, 3, 16);
-		}
-		if (npw == 6) {
-			if (vmode == 2) { if (center) WS_GO(4, 4, true, 2, 6, 32); else WS_GO(4, 4, false, 2, 6, 32); }
-			if (center) WS_GO(4, 4, true, 1, 6, 32); else WS_GO(4, 4, false, 1, 6, 32);
-		}
-		if (vmode == 2) { if (center) WS_GO(4, 4, true, 2, 4, 32); else WS_GO(4, 4, false, 2, 4, 32); }
-		if (center) WS_GO(4, 4, true, 1, 4, 32); else WS_GO(4, 4, false, 1, 4, 32);
-	}
-#undef WS_GO
+	if (halo <= 1) return launch_ws<1, 6>(*tm, hv, vol, out, D, H, W, ld, direction, s);
+	if (halo <= 4) return launch_ws<4, 4>(*tm, hv, vol, out, D, H, W, ld, direction, s);
 	return ADCENSUS_ELIMIT;
 }

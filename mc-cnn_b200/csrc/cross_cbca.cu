@@ -422,10 +422,8 @@ int launch_win(const uint32_t *a0, const uint32_t *a1, const float *vol, float *
 	// disparities per CTA.  Measured at 370x1226x228: 4..12 -> 1.01-1.04 ms, 16 -> 1.01 ms, 19 (whole
 	// waves) -> 1.08 ms: the kernel is issue-bound and balances dynamically, so the chunk size hardly
 	// matters; 10 keeps the per-chunk re-staging of the packed arms (L2 traffic only) small.
-	const char *env = getenv("ADCENSUS_CBCA_DCH");   // tuning knob, not part of the ABI
-	int dch = env ? atoi(env) : 10;
-	if (dch < 1) dch = 1;
-	if (dch > CW_DCH_MAX) dch = CW_DCH_MAX;
+	constexpr int dch = 10;
+	static_assert(dch <= CW_DCH_MAX, "arm window too narrow");
 	dim3 grid(adc_div_up(W, CW_TX), adc_div_up(H, CW_TY), adc_div_up(D, dch));
 	cbca_win_kernel<R><<<grid, CW_NT, SMEM, s>>>(a0, a1, vol, out, D, H, W, ld, direction, dch, gate, gate_lo, gate_hi);
 	return 0;

@@ -539,8 +539,7 @@ extern "C" int mccnn_feature_tower_forward(const mccnn_feature_tower *h, const f
 		p.taps_per_pass = FT_KA / h->fm;                       // K of a pass = taps x Cin <= 320
 		if (p.taps_per_pass > 9) p.taps_per_pass = 9;
 		const dim3 grid(adc_div_up(W, SH_M), H, nimg);
-		static const int resident_ok = getenv("ADCENSUS_TOWER_RESIDENT") ? atoi(getenv("ADCENSUS_TOWER_RESIDENT")) : 1;   // tuning knob
-		if (resident_ok && h->fm == 64) {                          // weights resident, persistent CTAs (the fast architecture)
+		if (h->fm == 64) {                                         // weights resident, persistent CTAs (the fast architecture)
 			static bool attr_r3[64] = {false}, attr_r1[64] = {false};
 			const int ntile = nimg * H * adc_div_up(W, SH_M);
 			const int nb = ntile < adc_num_sms() ? ntile : adc_num_sms();

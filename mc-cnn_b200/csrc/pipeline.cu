@@ -27,7 +27,7 @@ int adc_cbca_packed(const uint32_t *pk, const float *x0c, const float *x1c,
 		    const float *vol, float *out, int D, int H, int W, int ld, int direction, int maxlen, cudaStream_t s);
 size_t adc_packed_hv_words(int H, int W);
 int adc_pack_arms_hv(const float *xc, uint32_t *hv, int which, int H, int W, cudaStream_t s);
-int adc_cbca_tma_max_halo();
+int adc_cbca_ws_max_halo();
 void adc_cbca_tma_box(int halo, int *box_w, int *box_h);
 int adc_cbca_tma(const CUtensorMap *tm, const uint32_t *hv, const float *vol, float *out, int D, int H, int W, int ld, int direction,
 		 int halo, cudaStream_t s);
@@ -41,9 +41,7 @@ size_t adc_sgm_dhw_table_bytes(int H, int W, int D);
 int adc_sgm2_dhw(const float *x0, const float *x1, const float *in, float *acc, uint8_t *tab, int H, int W, int ld, int D,
 		 float pi1, float pi2, float tau_so, float alpha1, float q1, float q2, int direction, bool div4, cudaStream_t s);
 int adc_stereo_join(const float *input_L, const float *input_R, float *output_L, float *output_R,
-		    int C, int D, int H, int W, int ldo, int fast, const CUtensorMap *tmL, cudaStream_t s);
-int adc_stereo_join_dc(int D);
-int adc_stereo_join_fast_ok(const float *input_L, const float *input_R, const float *output_L, const float *output_R, int W, int ldo);
+		    int C, int D, int H, int W, int ldo, int fast, cudaStream_t s);
 int adc_fill_invalid(float *volL, float *volR, int D, int H, int W, int ld, cudaStream_t s);
 int adc_fix_border(float *vol, int D, int H, int W, int ld, int n, int direction, cudaStream_t s);
 int adc_argmin_pitched(const float *vol, float *disp, int D, int H, int W, int ld, cudaStream_t s);
@@ -73,9 +71,6 @@ struct mccnn_pipeline {
 	float *gauss;     // ks*ks
 	uint8_t *sgmtab;  // SGM penalty-class tables
 	int ks;
-	// tensor map of the left volume for StereoJoin's TMA store (box {128, 1, disparity chunk})
-	int sj_tm_ok;
-	CUtensorMap sj_tm;
 	// tensor maps of the volume buffers (inputs of the TMA-staged CBCA)
 	int ntm;
 	const float *tm_ptr[6];
@@ -118,7 +113,7 @@ int pipe_maxlen(const mccnn_pipeline *p) { return p->prm.L1 > 2 ? p->prm.L1 : 2;
 int add_tensor_map(mccnn_pipeline *p, const float *buf)
 {
 	const int halo = pipe_maxlen(p) - 1;
-	if (halo > adc_cbca_tma_max_halo()) return 0;      // such presets run the exact kernels
+	if (halo > adc_cbca_ws_max_halo()) return 0;       // such presets run the exact kernels
 	if (p->ntm >= 6) return ADCENSUS_EINVAL;
 	int bw, bh;
 	adc_cbca_tma_box(halo, &bw, &bh);
@@ -176,12 +171,6 @@ extern "C" int mccnn_pipeline_create(mccnn_pipeline **out, int C, int D, int H, 
 	if (!rc) rc = (int)cudaMemset(p->maxlen, 0, sizeof(int));
 	if (!rc) rc = dev_alloc((void **)&p->maps, 8 * p->HW * f, &p->bytes);
 	if (!rc) rc = dev_alloc((void **)&p->sgmtab, p->tab_bytes, &p->bytes);
-	if (!rc) {
-		const uint64_t dims[3] = {(uint64_t)W, (uint64_t)H, (uint64_t)D};
-		const uint64_t strides[2] = {(uint64_t)p->ld * 4, (uint64_t)p->ld * 4 * (uint64_t)H};
-		const uint32_t box[3] = {128u, 1u, (uint32_t)adc_stereo_join_dc(D)};
-		p->sj_tm_ok = adc_tma_encode(&p->sj_tm, p->vols, 3, dims, strides, box) == 0;
-	}
 	if (!rc) rc = add_tensor_map(p, p->vols);
 	if (!rc) rc = add_tensor_map(p, p->vols + p->V);
 	if (!rc) rc = add_tensor_map(p, p->bufA);
@@ -324,12 +313,8 @@ extern "C" int mccnn_pipeline_run(mccnn_pipeline *p, const float *featL, const f
 	int nl = 0;
 
 	float *volsL = p->vols, *volsR = p->vols + V;
-	// main.lua:946 (only what :947 leaves); on the fast path StereoJoin's TMA store fills the left volume's invalid entries itself
-	// (measured on B200 at K228: 0.51 ms against 0.45 ms for the plain path, so it is opt-in until it wins: ADCENSUS_SJ_FAST=1)
-	static const bool sj_fast_env = getenv("ADCENSUS_SJ_FAST") && atoi(getenv("ADCENSUS_SJ_FAST"));
-	const bool sj_fast = sj_fast_env && p->sj_tm_ok && adc_stereo_join_fast_ok(featL, featR, volsL, volsR, W, ld);
-	STEP(adc_fill_invalid(sj_fast ? nullptr : volsL, volsR, D, H, W, ld, s)); nl += 1;
-	STEP(adc_stereo_join(featL, featR, volsL, volsR, C, D, H, W, ld, sj_fast, sj_fast ? &p->sj_tm : nullptr, s)); nl += 1;   // :947
+	STEP(adc_fill_invalid(volsL, volsR, D, H, W, ld, s)); nl += 1;                                // main.lua:946 (only what :947 leaves)
+	STEP(adc_stereo_join(featL, featR, volsL, volsR, C, D, H, W, ld, /*fast=*/0, s)); nl += 1;    // :947
 	STEP(adc_fix_border(volsL, D, H, W, ld, o.border, -1, s));                                    // :948
 	STEP(adc_fix_border(volsR, D, H, W, ld, o.border, 1, s)); nl += o.border ? 2 : 0;             // :949
 
@@ -342,10 +327,7 @@ extern "C" int mccnn_pipeline_run(mccnn_pipeline *p, const float *featL, const f
 	// constant-work aggregation only for arms <= 5 (the KITTI presets, cbca_ws.cu): with the Middlebury presets' arms of up to
 	// 14 pixels the first-generation kernel's float prefixes over 27 x 27 windows reach 1.03e-4 after six iterations (measured,
 	// mb slow at 300 x 700 x 128) -- outside the 1e-4 contract -- so those presets run the exact tile kernels in every mode
-	// (ADCENSUS_CBCA_FAST_LONG=1 overrides)
-	static const bool fast_long = getenv("ADCENSUS_CBCA_FAST_LONG") && atoi(getenv("ADCENSUS_CBCA_FAST_LONG"));
-	const int fast_halo = fast_long ? adc_cbca_tma_max_halo() : 4;
-	const bool tma = p->cbca_mode && !nan_in_valid && maxlen - 1 <= fast_halo && p->ntm > 0;
+	const bool tma = p->cbca_mode && !nan_in_valid && maxlen - 1 <= adc_cbca_ws_max_halo();
 	uint32_t *hv = p->packed + adc_packed_words(H, W);
 	if (ncbca > 0) {
 		STEP(adcensus_cross(imgL, p->x0c, H, W, o.L1, o.tau1, s));

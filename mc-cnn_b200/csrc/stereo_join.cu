@@ -24,7 +24,6 @@
 // Roofline: 2*C*H*W*4 bytes read + 2*valid*4 bytes written (valid = H*(D*W -
 // D(D-1)/2)); at C=64 the FMA work (2*C flop per output) sits at the fp32 ridge
 // of the chip, so the kernel is tuned like a GEMM and reported against HBM.
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -332,10 +331,7 @@ int sj_ns(int D)
 // outputs (D, H, ldo) with row pitch ldo >= W (the fused pipeline's private volumes); features (C, H, W) contiguous.
 // The fast load / store path needs W even, 8-byte aligned features and 16-byte aligned outputs with ldo % 4 == 0; it
 // writes NaN into the left volume's entries x < d (no separate fill needed there; hence opt-in through `fast`: the
-// operator itself leaves them untouched, adcensus.cu:1467) and leaves the right volume's invalid entries untouched.  tmL: tensor map of output_L with box {128, 1, adc_stereo_join_dc(D)}
-// (NULL: encoded here).
-int adc_stereo_join_dc(int D) { return 16 * sj_ns(D) - 8; }
-
+// operator itself leaves them untouched, adcensus.cu:1467) and leaves the right volume's invalid entries untouched.
 int adc_stereo_join_fast_ok(const float *input_L, const float *input_R, const float *output_L, const float *output_R, int W, int ldo)
 {
 	return (W % 2 == 0) && (ldo % 4 == 0) && ((((uintptr_t)input_L) | ((uintptr_t)input_R)) % 8 == 0) &&
@@ -343,26 +339,22 @@ int adc_stereo_join_fast_ok(const float *input_L, const float *input_R, const fl
 }
 
 int adc_stereo_join(const float *input_L, const float *input_R, float *output_L, float *output_R,
-		    int C, int D, int H, int W, int ldo, int fast, const CUtensorMap *tmL, cudaStream_t s)
+		    int C, int D, int H, int W, int ldo, int fast, cudaStream_t s)
 {
 	if (!input_L || !input_R || !output_L || !output_R) return ADCENSUS_EINVAL;
 	if (C < 1 || D < 1 || H < 1 || W < 1 || H > 65535 || ldo < W) return ADCENSUS_EINVAL;
 	if (C > 128) return ADCENSUS_ELIMIT;  // reference: float L_cache[128] (adcensus.cu:1460-1461)
 	const int ns = sj_ns(D);
-	static const int use_tma = getenv("ADCENSUS_SJ_TMA") ? atoi(getenv("ADCENSUS_SJ_TMA")) : 1;   // tuning knob
-	if (use_tma && !fast && adc_stereo_join_tma_ok(input_L, input_R, output_L, output_R, H, W) && (ldo % 4 == 0 || ldo == W))
+	if (!fast && adc_stereo_join_tma_ok(input_L, input_R, output_L, output_R, H, W) && (ldo % 4 == 0 || ldo == W))
 		return adc_stereo_join_tma(input_L, input_R, output_L, output_R, C, D, H, W, ldo, ns, s);
 	if (fast && adc_stereo_join_fast_ok(input_L, input_R, output_L, output_R, W, ldo)) {
-		CUtensorMap local;
-		if (!tmL) {
-			const uint64_t dims[3] = {(uint64_t)W, (uint64_t)H, (uint64_t)D};
-			const uint64_t strides[2] = {(uint64_t)ldo * 4, (uint64_t)ldo * 4 * (uint64_t)H};
-			const uint32_t box[3] = {(uint32_t)SJ_TX, 1u, (uint32_t)(16 * ns - 8)};
-			int rc = adc_tma_encode(&local, output_L, 3, dims, strides, box);
-			if (rc) return rc;
-			tmL = &local;
-		}
-		return dispatch<true>(ns, *tmL, input_L, input_R, output_L, output_R, C, D, H, W, ldo, s);
+		CUtensorMap tmL;
+		const uint64_t dims[3] = {(uint64_t)W, (uint64_t)H, (uint64_t)D};
+		const uint64_t strides[2] = {(uint64_t)ldo * 4, (uint64_t)ldo * 4 * (uint64_t)H};
+		const uint32_t box[3] = {(uint32_t)SJ_TX, 1u, (uint32_t)(16 * ns - 8)};
+		int rc = adc_tma_encode(&tmL, output_L, 3, dims, strides, box);
+		if (rc) return rc;
+		return dispatch<true>(ns, tmL, input_L, input_R, output_L, output_R, C, D, H, W, ldo, s);
 	}
 	CUtensorMap dummy;
 	memset(&dummy, 0, sizeof(dummy));
@@ -372,7 +364,7 @@ int adc_stereo_join(const float *input_L, const float *input_R, float *output_L,
 extern "C" int adcensus_StereoJoin(const float *input_L, const float *input_R, float *output_L, float *output_R,
 				   int C, int D, int H, int W, adcensus_stream_t stream)
 {
-	return adc_stereo_join(input_L, input_R, output_L, output_R, C, D, H, W, W, /*fast=*/0, nullptr, adc_stream(stream));
+	return adc_stereo_join(input_L, input_R, output_L, output_R, C, D, H, W, W, /*fast=*/0, adc_stream(stream));
 }
 
 // StereoJoin into pitched (D, H, ld) volumes (the fused pipeline's private layout).  Unlike the operator above this
@@ -383,5 +375,5 @@ extern "C" int mccnn_stereo_join_pitched(const float *input_L, const float *inpu
 {
 	if (!input_L || !input_R || !output_L || !output_R || ld < W) return ADCENSUS_EINVAL;
 	if (!adc_stereo_join_fast_ok(input_L, input_R, output_L, output_R, W, ld)) return ADCENSUS_EINVAL;
-	return adc_stereo_join(input_L, input_R, output_L, output_R, C, D, H, W, ld, /*fast=*/1, nullptr, adc_stream(stream));
+	return adc_stereo_join(input_L, input_R, output_L, output_R, C, D, H, W, ld, /*fast=*/1, adc_stream(stream));
 }

@@ -1,7 +1,6 @@
 """Fast (constant-work) CBCA against the exact mode at the bench size on a structured synthetic pair: max relative error of
 the final left volume and the fraction of disparity-map pixels that differ by more than 1e-4 (the exact mode is
-bit-identical to the reference, tests/test_gpu_parity.py).  Kernel variants are chosen by environment variables
-(ADCENSUS_CBCA_WS / _VMODE / _CENTER), read once per process."""
+bit-identical to the reference, tests/test_gpu_parity.py)."""
 import argparse
 import os
 import sys
@@ -38,6 +37,5 @@ nanok = bool((torch.isnan(ve) == torch.isnan(vf)).all())
 m = ~torch.isnan(ve)
 err = ((vf[m] - ve[m]).abs() / ve[m].abs().clamp(min=1.0))
 frac = float(((df - de).abs() > 1e-4 * de.abs().clamp(min=1.0)).float().mean())
-print("env WS=%s VMODE=%s CENTER=%s: nan_pattern_ok=%s vol max_rel_err=%.3g mean_rel_err=%.3g disp_frac_off=%.3g"
-      % (os.environ.get("ADCENSUS_CBCA_WS", "-"), os.environ.get("ADCENSUS_CBCA_VMODE", "-"), os.environ.get("ADCENSUS_CBCA_CENTER", "-"),
-         nanok, float(err.max()), float(err.mean()), frac))
+print("nan_pattern_ok=%s vol max_rel_err=%.3g mean_rel_err=%.3g disp_frac_off=%.3g"
+      % (nanok, float(err.max()), float(err.mean()), frac))

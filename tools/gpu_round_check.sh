@@ -15,11 +15,8 @@ mkdir -p $OUT
 date
 python -m pytest tests -m gpu -q 2>&1 | tail -5 | tee $OUT/${TAG}_pytest.log
 python -c "import __graft_entry__ as g; g.smoke(); print('smoke ok')" 2>&1 | tail -1
-# experimental kernels (opt-in, env-gated tests): validate and time them in the same call
-MCCNN_EXPERIMENTAL=1 python -m pytest tests/test_gpu_parity.py -m gpu -q -k experimental 2>&1 | tail -4 | tee $OUT/${TAG}_pytest_experimental.log
 python tools/time_pipeline.py 2>&1 | tail -1
-python tools/time_pipeline.py --fast 2>&1 | tail -1
-python tools/time_pipeline.py --fast-level 2 2>&1 | tail -1
+python tools/time_pipeline.py --exact 2>&1 | tail -1
 python bench.py > $OUT/${TAG}_bench_n1.json 2> $OUT/${TAG}_bench_n1.err
 cut -c1-220 $OUT/${TAG}_bench_n1.json
 python bench.py --impl reference > $OUT/${TAG}_bench_reference_n1.json 2> /dev/null

@@ -1,6 +1,6 @@
 """Time the fused pipeline (device-resident inputs) at the bench workload: prints ms per pair.
 
-    ADCENSUS_CBCA_DCH=14 python tools/time_pipeline.py [--iters 10] [--fast]
+    python tools/time_pipeline.py [--iters 10] [--exact]
 """
 import argparse
 import os
