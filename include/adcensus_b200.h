@@ -13,7 +13,7 @@
  * Conventions
  *   - every pointer is a DEVICE pointer to contiguous float32 (the reference
  *     ignores strides: raw THCudaTensor_data + sizes);
- *   - shapes: features (C,H,W); cost volumes (D,H,W); SGM volumes (H,W,D); `*_pitched` / `*_dhw` entry points take
+ *   - shapes: features (C,H,W); cost volumes (D,H,W); SGM volumes (H,W,D); `*_pitched` entry points take
  *     (D,H,ld) volumes with a row pitch ld (the fused pipeline's private layout);
  *     images / disparity maps (H,W); cross arms (4,H,W);
  *   - `stream` is a cudaStream_t (0 = legacy default stream, what the
@@ -114,14 +114,6 @@ int mccnn_cbca_fast_pitched_packed(const void *hv, const float *vol_in, float *v
 int adcensus_sgm2(const float *x0, const float *x1, const float *input, float *output, float *tmp,
 		  int H, int W, int D, float pi1, float pi2, float tau_so, float alpha1,
 		  float sgm_q1, float sgm_q2, int direction, adcensus_stream_t stream);
-
-/* sgm2 on pitched (D, H, ld) volumes, no permutes (csrc/sgm_dhw.cu): output = sum of the four directional costs of
- * input (right, left, down, up: the reference's accumulation order, bit-identical values), times 1/4 when div4 != 0
- * (main.lua:1008-1020 in one call).  ld % 4 == 0, ld >= W rounded up to 4, 16-byte aligned bases; output need not be
- * initialised and its padding columns receive unspecified values. */
-int mccnn_sgm2_dhw(const float *x0, const float *x1, const float *input, float *output,
-		   int H, int W, int ld, int D, float pi1, float pi2, float tau_so, float alpha1,
-		   float sgm_q1, float sgm_q2, int direction, int div4, adcensus_stream_t stream);
 
 /* Band-wise sgm2 for the row-band / column-band multi-GPU split: x0, x1 are the FULL Ht x Wt images,
  * input/output this GPU's band volume (H,W,D) at image offset (yoff, xoff); pass_mask selects scan
@@ -242,10 +234,6 @@ size_t mccnn_pipeline_device_bytes(const mccnn_pipeline *p);
 void mccnn_pipeline_set_cbca_mode(mccnn_pipeline *p, int mode);
 int mccnn_pipeline_get_cbca_mode(const mccnn_pipeline *p);
 void mccnn_pipeline_set_fast_cbca(mccnn_pipeline *p, int on);
-/* SGM data layout inside the pipeline: 0 (default) = permute the pitched volume to (H,W,D) and back around sgm2 like
- * main.lua:1008-1020 (fused /4); 1 = scan the (D,H,ld) layout directly (mccnn_sgm2_dhw, no permutes).  Bit-identical
- * results either way; ADCENSUS_SGM_DHW=1 in the environment makes 1 the default. */
-void mccnn_pipeline_set_sgm_layout(mccnn_pipeline *p, int dhw);
 /* opt-in: run the two directions of main.lua:955 concurrently (0 = off: one stream, 4V of volume buffers;
  * 1 = direction -1 on a side stream with its own 2V + tables, started when direction +1 reaches its SGM phase;
  * 2 = additionally the permute / SGM phases on high-priority streams).  Results are identical in every mode

@@ -14,7 +14,7 @@ CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 OBJDIR = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libadcensus_b200.so")
-SOURCES = ["common.cu", "stereo_join.cu", "stereo_join_tma.cu", "cross_cbca.cu", "cbca_tma.cu", "cbca_ws.cu", "sgm.cu", "sgm_dhw.cu", "post.cu", "adcensus_cost.cu", "scorer_head.cu", "feature_tower.cu", "pipeline.cu"]
+SOURCES = ["common.cu", "stereo_join.cu", "stereo_join_tma.cu", "cross_cbca.cu", "cbca_tma.cu", "cbca_ws.cu", "sgm.cu", "post.cu", "adcensus_cost.cu", "scorer_head.cu", "feature_tower.cu", "pipeline.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 NVCC_FLAGS = ARCH + ["-O3", "-lineinfo", "-diag-suppress", "177", "-std=c++17", "--compiler-options", "-fPIC", "-I" + INCLUDE, "-I" + CSRC]
 
@@ -63,7 +63,8 @@ def build(force=False, verbose=False):
                 sys.stderr.write(log)
     objs = [os.path.join(OBJDIR, src.replace(".cu", ".o")) for src in SOURCES]
     if force or jobs or not os.path.exists(LIB):
-        cmd = [nvcc] + ARCH + ["--shared", "-o", LIB] + objs + ["-lcudart"]
+        # --no-undefined: an internal reference without a definition fails here rather than at the first dlopen
+        cmd = [nvcc] + ARCH + ["--shared", "-Xlinker", "--no-undefined", "-o", LIB] + objs + ["-lcudart"]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError("link failed:\n%s\n%s" % (r.stdout, r.stderr))

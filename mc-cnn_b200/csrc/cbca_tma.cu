@@ -26,8 +26,7 @@
 //     ring of 2R + 2 rows; the output of row y is emitted R rows later from two ring reads.
 // Arms are pre-packed per image into H words (4L | 4(R-1) << 16) and V words (U << 8 | D << 24), lengths
 // relative to the pixel, so "max of left ends / min of right ends" is one packed 16-bit minimum.
-#include "common.cuh"
-#include "tma.cuh"
+#include "internal.cuh"
 
 namespace {
 
@@ -344,14 +343,8 @@ int adc_pack_arms_hv(const float *xc, uint32_t *hv, int which, int H, int W, cud
 	return 0;
 }
 
-// second-generation kernel for short arms (cbca_ws.cu)
-int adc_cbca_ws_max_halo();
-void adc_cbca_ws_box(int halo, int *box_w, int *box_h);
-int adc_cbca_ws(const CUtensorMap *tm, const uint32_t *hv, const float *vol, float *out, int D, int H, int W, int ld, int direction,
-		int halo, cudaStream_t s);
-
 // largest support radius (longest arm - 1) the constant-work kernel is instantiated for
-int adc_cbca_tma_max_halo() { return 13; }
+static int adc_cbca_tma_max_halo() { return 13; }
 
 // box of the tensor map a volume needs for support radius `halo` (= longest arm - 1)
 void adc_cbca_tma_box(int halo, int *box_w, int *box_h)

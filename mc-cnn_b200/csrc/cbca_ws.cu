@@ -24,8 +24,7 @@
 // shared-memory wavefronts per output, 64-row tiles (halo overhead 1.25 instead of 1.4 / 1.5), and centred prefixes.
 // NOT bit-exact by construction (1e-4 contract; measured ~1e-7).
 // Arms up to 5 pixels (R <= 4, the KITTI presets); longer arms stay on cbca_tma.cu / the exact kernels.
-#include "common.cuh"
-#include "tma.cuh"
+#include "internal.cuh"
 
 namespace {
 

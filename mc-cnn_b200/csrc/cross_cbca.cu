@@ -23,7 +23,7 @@
 // by HBM -- see DESIGN.md.
 #include <stdlib.h>
 
-#include "common.cuh"
+#include "internal.cuh"
 
 namespace {
 

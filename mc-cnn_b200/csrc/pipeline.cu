@@ -17,35 +17,7 @@
 #include <stdlib.h>
 #include <string.h>
 
-#include "common.cuh"
-#include "tma.cuh"
-
-// internal entry points of the other translation units
-size_t adc_packed_words(int H, int W);
-int adc_pack_arms(const float *xc, uint32_t *pk, int which, int H, int W, int *maxlen_dev, cudaStream_t s);
-int adc_cbca_packed(const uint32_t *pk, const float *x0c, const float *x1c,
-		    const float *vol, float *out, int D, int H, int W, int ld, int direction, int maxlen, cudaStream_t s);
-size_t adc_packed_hv_words(int H, int W);
-int adc_pack_arms_hv(const float *xc, uint32_t *hv, int which, int H, int W, cudaStream_t s);
-int adc_cbca_ws_max_halo();
-void adc_cbca_tma_box(int halo, int *box_w, int *box_h);
-int adc_cbca_tma(const CUtensorMap *tm, const uint32_t *hv, const float *vol, float *out, int D, int H, int W, int ld, int direction,
-		 int halo, cudaStream_t s);
-size_t adc_sgm_table_bytes(int H, int W, int D);
-int adc_sgm2(const float *x0, const float *x1, const float *in, float *out, uint8_t *tab, int H, int W, int D,
-	     float pi1, float pi2, float tau_so, float alpha1, float q1, float q2, int direction,
-	     bool zero_out, cudaStream_t s);
-int adc_transpose_dhw_pitched_to_hwd(const float *in, float *out, int D, int H, int W, int ld, cudaStream_t s);
-int adc_transpose_hwd_to_dhw_pitched_div4(const float *in, float *out, int D, int H, int W, int ld, cudaStream_t s);
-size_t adc_sgm_dhw_table_bytes(int H, int W, int D);
-int adc_sgm2_dhw(const float *x0, const float *x1, const float *in, float *acc, uint8_t *tab, int H, int W, int ld, int D,
-		 float pi1, float pi2, float tau_so, float alpha1, float q1, float q2, int direction, bool div4, cudaStream_t s);
-int adc_stereo_join(const float *input_L, const float *input_R, float *output_L, float *output_R,
-		    int C, int D, int H, int W, int ldo, int fast, cudaStream_t s);
-int adc_fill_invalid(float *volL, float *volR, int D, int H, int W, int ld, cudaStream_t s);
-int adc_fix_border(float *vol, int D, int H, int W, int ld, int n, int direction, cudaStream_t s);
-int adc_argmin_pitched(const float *vol, float *disp, int D, int H, int W, int ld, cudaStream_t s);
-int adc_subpixel(const float *d0, const float *c2, float *out, int H, int W, int ld, int disp_max, cudaStream_t s);
+#include "internal.cuh"
 
 // Private volume layout: (D, H, ld), ld = W rounded up to a multiple of 4 floats.  Every row then starts on a
 // 16-byte boundary: tensor maps (TMA) can describe the volumes, and 16-byte vector / cp.async accesses along x are
@@ -58,7 +30,6 @@ struct mccnn_pipeline {
 	size_t bytes;
 	int launches;
 	int cbca_mode;    // 1 = constant-work aggregation (default, 1e-4 contract), 0 = exact (bit-identical to the reference)
-	int sgm_dhw;      // 1 = scan the (D,H,ld) layout directly (sgm_dhw.cu, no permutes); 0 (default) = permute to (H,W,D) like main.lua:1008
 	size_t tab_bytes;
 	// device buffers
 	float *vols;      // 2V: [0] left volume, [1] right volume (main.lua:946)
@@ -155,10 +126,7 @@ extern "C" int mccnn_pipeline_create(mccnn_pipeline **out, int C, int D, int H, 
 	p->V = (long)D * H * p->ld;
 	const char *ex = getenv("ADCENSUS_CBCA_EXACT");
 	p->cbca_mode = (ex && atoi(ex)) ? 0 : 1;
-	const char *sd = getenv("ADCENSUS_SGM_DHW");
-	p->sgm_dhw = (sd && atoi(sd)) ? 1 : 0;
 	p->tab_bytes = adc_sgm_table_bytes(H, W, D);
-	if (adc_sgm_dhw_table_bytes(H, W, D) > p->tab_bytes) p->tab_bytes = adc_sgm_dhw_table_bytes(H, W, D);
 	int rc = 0;
 	const size_t f = sizeof(float);
 	if (!rc) rc = dev_alloc((void **)&p->vols, 2 * p->V * f, &p->bytes);
@@ -230,8 +198,6 @@ extern "C" size_t mccnn_pipeline_device_bytes(const mccnn_pipeline *p) { return 
 extern "C" void mccnn_pipeline_set_cbca_mode(mccnn_pipeline *p, int mode) { if (p) p->cbca_mode = mode ? 1 : 0; }
 extern "C" int mccnn_pipeline_get_cbca_mode(const mccnn_pipeline *p) { return p ? p->cbca_mode : -1; }
 extern "C" void mccnn_pipeline_set_fast_cbca(mccnn_pipeline *p, int on) { mccnn_pipeline_set_cbca_mode(p, on); }
-// 0 (default): permute to (H,W,D) for sgm2 like main.lua:1008; 1: scan (D,H,ld) directly (sgm_dhw.cu).  Same results.
-extern "C" void mccnn_pipeline_set_sgm_layout(mccnn_pipeline *p, int dhw) { if (p) p->sgm_dhw = dhw ? 1 : 0; }
 static void overlap_release(mccnn_pipeline *p)
 {
 	const size_t f = sizeof(float);
@@ -367,18 +333,11 @@ extern "C" int mccnn_pipeline_run(mccnn_pipeline *p, const float *featL, const f
 			STEP((int)cudaStreamWaitEvent(ss, p->ev_hi_in[k], 0));
 		}
 		for (int it = 0; it < o.sgm_i; it++) {                                                   // :1008-1020
-			if (p->sgm_dhw) {                                                                    // no permutes: (D,H,ld) scans
-				STEP(adc_sgm2_dhw(imgL, imgR, cur, acc, tab, H, W, ld, D, o.pi1, o.pi2, o.tau_so, o.alpha1,
-						  o.sgm_q1, o.sgm_q2, direction, /*div4=*/true, ss));              // :1014-1016, :1020
-				float *t = cur; cur = acc; acc = t;
-				nl += 5;
-			} else {
-				STEP(adc_transpose_dhw_pitched_to_hwd(cur, spare, D, H, W, ld, ss));             // :1008
-				STEP(adc_sgm2(imgL, imgR, spare, acc, tab, H, W, D, o.pi1, o.pi2, o.tau_so, o.alpha1,
-					      o.sgm_q1, o.sgm_q2, direction, /*zero_out=*/true, ss));                // :1014-1016
-				STEP(adc_transpose_hwd_to_dhw_pitched_div4(acc, cur, D, H, W, ld, ss));          // :1017-1020
-				nl += 7;
-			}
+			STEP(adc_transpose_dhw_pitched_to_hwd(cur, spare, D, H, W, ld, ss));                 // :1008
+			STEP(adc_sgm2(imgL, imgR, spare, acc, tab, H, W, D, o.pi1, o.pi2, o.tau_so, o.alpha1,
+				      o.sgm_q1, o.sgm_q2, direction, /*zero_out=*/true, ss));                    // :1014-1016
+			STEP(adc_transpose_hwd_to_dhw_pitched_div4(acc, cur, D, H, W, ld, ss));              // :1017-1020
+			nl += 7;
 		}
 		if (ss != ds) {
 			STEP((int)cudaEventRecord(p->ev_hi_out[k], ss));
@@ -469,7 +428,6 @@ static int batch_lanes(mccnn_pipeline *p, mccnn_pipeline **lane, int want)
 		}
 		q = q->twin;
 		q->cbca_mode = p->cbca_mode;
-		q->sgm_dhw = p->sgm_dhw;
 		if (q->overlap != p->overlap) mccnn_pipeline_set_overlap(q, p->overlap);
 		lane[n] = q;
 	}

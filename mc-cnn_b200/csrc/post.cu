@@ -9,7 +9,7 @@
 // (torch.min).  All of these are bit-exact restatements: index/label work is
 // integer, the float expressions keep the reference's operation order (fmaf where
 // nvcc contracts the reference's `a += b * c`).
-#include "common.cuh"
+#include "internal.cuh"
 
 namespace {
 
@@ -460,7 +460,7 @@ int adc_transpose_hwd_to_dhw_pitched_div4(const float *in, float *out, int D, in
 	return 0;
 }
 
-int adc_transpose(const float *in, float *out, long R, long Cn, float div, bool do_div, cudaStream_t s)
+static int adc_transpose(const float *in, float *out, long R, long Cn, float div, bool do_div, cudaStream_t s)
 {
 	const bool vec = (R % 4 == 0) && (Cn % 4 == 0) && ((((uintptr_t)in) | ((uintptr_t)out)) % 16 == 0);
 	const int tile = vec ? 64 : 32;

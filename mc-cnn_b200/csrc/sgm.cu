@@ -34,7 +34,7 @@
 // Algorithmic traffic per call: 4 passes x (read input + read-modify-write
 // output) = 12V bytes (V = 4*D*H*W); 11V when the caller guarantees a zeroed
 // output (pipeline), because the first pass then skips the read.
-#include "common.cuh"
+#include "internal.cuh"
 
 namespace {
 
@@ -601,7 +601,7 @@ static int sgm_slots(int D) { return D <= 32 ? 32 : (D <= 64 ? 64 : (D <= 128 ? 
 // four byte-class planes + the selector words of the vertical scans (128 bytes per pixel)
 size_t adc_sgm_table_bytes(int H, int W, int D) { return sgm_sel_offset(H, W + 2 * sgm_slots(D)) + (size_t)128 * H * W; }
 
-int adc_sgm_classes(const float *x0, const float *x1, uint8_t *tab, int Ht, int Wt, int D, float tau_so, cudaStream_t s)
+static int adc_sgm_classes(const float *x0, const float *x1, uint8_t *tab, int Ht, int Wt, int D, float tau_so, cudaStream_t s)
 {
 	const int pad = sgm_slots(D);
 	const long plane = (long)Ht * (Wt + 2 * pad);
@@ -614,7 +614,7 @@ int adc_sgm_classes(const float *x0, const float *x1, uint8_t *tab, int Ht, int 
 // Ht x Wt image whose class tables are in `tab` (adc_sgm_classes).  zero_out: `output` is known
 // to be all zeros (main.lua:1014) -> the first (rightward) pass skips reading it.
 // selector words of the vertical scans for the W columns at image offset xoff (all Ht table rows) and one `direction`
-int adc_sgm_selectors(uint8_t *tab, int W, int D, int Ht, int Wt, int xoff, int direction, cudaStream_t s)
+static int adc_sgm_selectors(uint8_t *tab, int W, int D, int Ht, int Wt, int xoff, int direction, cudaStream_t s)
 {
 	const int pad = sgm_slots(D);
 	unsigned *sel = reinterpret_cast<unsigned *>(tab + sgm_sel_offset(Ht, Wt + 2 * pad));
@@ -633,9 +633,9 @@ int adc_sgm_selectors(uint8_t *tab, int W, int D, int Ht, int Wt, int xoff, int 
 
 // the selected passes with tables (and, for vertical passes, selectors) already built; vertical passes may cover the
 // columns [xa, xb) only and carry the line state across row bands (state_in / state_out, [W][32K] floats, NULL = border)
-int adc_sgm2_passes(const float *in, float *out, const uint8_t *tab, int H, int W, int D, int Ht, int Wt, int yoff, int xoff,
-		    float pi1, float pi2, float tau_so, float alpha1, float q1, float q2, int direction,
-		    bool zero_out, int pass_mask, int xa, int xb, const float *state_in, float *state_out, cudaStream_t s)
+static int adc_sgm2_passes(const float *in, float *out, const uint8_t *tab, int H, int W, int D, int Ht, int Wt, int yoff, int xoff,
+			   float pi1, float pi2, float tau_so, float alpha1, float q1, float q2, int direction,
+			   bool zero_out, int pass_mask, int xa, int xb, const float *state_in, float *state_out, cudaStream_t s)
 {
 	SgmParams prm{pi1, pi2, tau_so, alpha1, q1, q2, direction, Ht, Wt, yoff, xoff, state_in, state_out, xa, xb};
 	const int pad = sgm_slots(D);
@@ -650,9 +650,9 @@ int adc_sgm2_passes(const float *in, float *out, const uint8_t *tab, int H, int 
 		   : launch_all<16, false>(tab, in, out, H, W, D, pad, prm, zero_out, pass_mask, s);
 }
 
-int adc_sgm2_band(const float *in, float *out, const uint8_t *tab, int H, int W, int D, int Ht, int Wt, int yoff, int xoff,
-		  float pi1, float pi2, float tau_so, float alpha1, float q1, float q2, int direction,
-		  bool zero_out, int pass_mask, cudaStream_t s)
+static int adc_sgm2_band(const float *in, float *out, const uint8_t *tab, int H, int W, int D, int Ht, int Wt, int yoff, int xoff,
+			 float pi1, float pi2, float tau_so, float alpha1, float q1, float q2, int direction,
+			 bool zero_out, int pass_mask, cudaStream_t s)
 {
 	if (pass_mask & 12) {                              // vertical scans: band = whole columns (H == Ht)
 		int rc = adc_sgm_selectors(const_cast<uint8_t *>(tab), W, D, Ht, Wt, xoff, direction, s);

@@ -26,8 +26,7 @@
 // of the chip, so the kernel is tuned like a GEMM and reported against HBM.
 #include <string.h>
 
-#include "common.cuh"
-#include "tma.cuh"
+#include "internal.cuh"
 
 namespace {
 
@@ -52,13 +51,6 @@ __device__ __forceinline__ unsigned long long sj_fma2(unsigned long long a, unsi
 	asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
 	return d;
 }
-
-}  // namespace
-// second generation (stereo_join_tma.cu): TMA-staged feature rows
-int adc_stereo_join_tma_ok(const float *input_L, const float *input_R, const float *output_L, const float *output_R, int H, int W);
-int adc_stereo_join_tma(const float *input_L, const float *input_R, float *output_L, float *output_R,
-			int C, int D, int H, int W, int ldo, int ns, cudaStream_t s);
-namespace {
 
 template <int NS>
 struct SJCfg {
@@ -332,7 +324,7 @@ int sj_ns(int D)
 // The fast load / store path needs W even, 8-byte aligned features and 16-byte aligned outputs with ldo % 4 == 0; it
 // writes NaN into the left volume's entries x < d (no separate fill needed there; hence opt-in through `fast`: the
 // operator itself leaves them untouched, adcensus.cu:1467) and leaves the right volume's invalid entries untouched.
-int adc_stereo_join_fast_ok(const float *input_L, const float *input_R, const float *output_L, const float *output_R, int W, int ldo)
+static int adc_stereo_join_fast_ok(const float *input_L, const float *input_R, const float *output_L, const float *output_R, int W, int ldo)
 {
 	return (W % 2 == 0) && (ldo % 4 == 0) && ((((uintptr_t)input_L) | ((uintptr_t)input_R)) % 8 == 0) &&
 	       ((((uintptr_t)output_L) | ((uintptr_t)output_R)) % 16 == 0);

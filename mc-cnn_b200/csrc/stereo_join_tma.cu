@@ -23,8 +23,7 @@
 //     selects cost more instructions than the 4-byte stores they saved).
 #include <string.h>
 
-#include "common.cuh"
-#include "tma.cuh"
+#include "internal.cuh"
 
 namespace {
 

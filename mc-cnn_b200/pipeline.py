@@ -201,10 +201,6 @@ class StereoPipeline:
     def cbca_mode(self):
         return "fast" if adcensus.lib().mccnn_pipeline_get_cbca_mode(self._h) else "exact"
 
-    def set_sgm_layout(self, dhw):
-        """True: sgm2 scans the (D,H,ld) layout directly (csrc/sgm_dhw.cu); False (default): permutes around sgm2 as main.lua does"""
-        adcensus.lib().mccnn_pipeline_set_sgm_layout(self._h, int(bool(dhw)))
-
     def set_fast_cbca(self, on=True):
         """older name of :meth:`set_cbca_mode`"""
         self.set_cbca_mode(1 if on else 0)

@@ -8,6 +8,7 @@ the reference's fp32 operation order, so the float volumes are required to be
 bit-identical too (NaN positions included), which is stricter than the 1e-4 the
 north star allows.
 """
+import ctypes
 import glob
 import os
 
@@ -197,6 +198,24 @@ def test_transposes_argmin(oracle):
     out = torch.empty((1, 1, H, W), device=dev())
     adcensus.spatial_argmin(cu(vol)[None], out)
     same(out, oracle.spatial_argmin(vol), "spatial_argmin")
+    # the pipeline's pitched (D, H, ld) forms, ld > W with garbage in the padding columns; D = 12 takes the 16-byte
+    # vector path (D % 4 == 0) that reads and writes the row padding, D = 13 the scalar one
+    vp = lambda t_: ctypes.c_void_p(t_.data_ptr())
+    for v in (vol[:12], vol):
+        Dv, ld = v.shape[0], (W + 3) // 4 * 4 + 4
+        pv = torch.full((Dv, H, ld), 777.0, device=dev())
+        pv[:, :, :W] = cu(v)
+        hwd = torch.full((H, W, Dv), -1.0, device=dev())
+        back = torch.full((Dv, H, ld), 777.0, device=dev())
+        disp = torch.full((H, W), -1.0, device=dev())
+        s = adcensus._stream(pv)
+        assert adcensus.lib().mccnn_transpose_dhw_pitched_to_hwd(vp(pv), vp(hwd), Dv, H, W, ld, s) == 0
+        assert adcensus.lib().mccnn_transpose_hwd_to_dhw_pitched_div4(vp(hwd), vp(back), Dv, H, W, ld, s) == 0
+        assert adcensus.lib().mccnn_argmin_pitched(vp(pv), vp(disp), Dv, H, W, ld, s) == 0
+        torch.cuda.synchronize()
+        same(hwd, oracle.transpose_dhw_to_hwd(v), "pitched transpose, D = %d" % Dv)
+        same(back[:, :, :W], v / 4, "pitched transpose back /4, D = %d" % Dv)
+        same(disp, oracle.spatial_argmin(v) - 1, "pitched argmin, D = %d" % Dv)
     # ties -> first index
     tie = np.zeros((4, 3, 5), np.float32)
     same(adcensus.argmin(cu(tie)[None]), np.zeros((3, 5), np.float32), "argmin ties")
